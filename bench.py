@@ -76,6 +76,11 @@ def parse():
         ap.add_argument("--" + name, type=typ, default=None, help="override the preset")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="bounded CPU-baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the answers of the last timed step as DIR/<name>.npy (ids, distances, counts, rows), at "
+                         "most 64 MB; for comparing two builds run with the same arguments.  Only rank 0's answers: with "
+                         "--gpus N that is its shard of the step.  The two --impl arms search different query batches in "
+                         "their last step, so their dumps do not line up row for row")
     a = ap.parse_args()
     preset = PRESETS[a.config]
     a.custom = False
@@ -92,6 +97,8 @@ def parse():
         a.steps = 5 if big else 100
     if a.warmup is None:
         a.warmup = 3 if big else 10
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     a.strong = big
     return a
 
@@ -179,6 +186,38 @@ def recall_stats(ids, dists, counts, t_ids, t_d):
     return rid / t_ids.shape[0], rball / t_ids.shape[0]
 
 
+DUMP_LIMIT = 64 * 1000 * 1000     # bytes, .npy headers included
+DUMP_HEADERS = 4096               # reserved for the four .npy headers (128 bytes each in practice)
+
+
+def step_slot(i, gstep, ngrp):
+    """(group, position in group) of the answer buffer timed step i writes: groups of gstep steps, ngrp groups rotating"""
+    return (i // gstep) % ngrp, i % gstep
+
+
+def decode_records(rec):
+    """Neighbour_api[nq][k] records (uint8 [nq, k, 16]: u64 origin id at byte 0, f32 distance at byte 8, the internal id
+    in the tail padding) -> (ids u64 [nq, k], distances f32 [nq, k])"""
+    rec = np.ascontiguousarray(rec, np.uint8)
+    return rec.view(np.uint64)[..., 0], rec.view(np.float32)[..., 2]
+
+
+def dump_outputs(out_dir, ids, dists, counts):
+    """Writes one step's answers as out_dir/{ids,distances,counts,rows}.npy (ids as float64: exact below 2**53; the
+    kernels pad unused slots with id 2**64-1, distance inf).  rows holds the query row numbers: all of them, or, when
+    the files would exceed DUMP_LIMIT bytes, a fixed seeded sample."""
+    nq, k = ids.shape
+    rows = np.arange(nq)
+    keep = (DUMP_LIMIT - DUMP_HEADERS) // (k * 8 + k * 4 + 4 + 8)
+    if nq > keep:
+        rows = np.sort(np.random.default_rng(0).choice(nq, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"ids": ids[rows].astype(np.float64), "distances": dists[rows].astype(np.float32),
+           "counts": counts[rows].astype(np.float32), "rows": rows.astype(np.float64)}
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 
 def workload_name(a, world=1):
     per = a.nq // world if a.strong else a.nq
@@ -239,7 +278,6 @@ def run_reference(a, rank, world):
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import pyoracle as po
     pkg = importlib.import_module("hnswlib-rs_b200")
-    po.build()
     cores = os.cpu_count() or 1
     X = pkg.datagen.make(a.data, a.n, a.d, 1)
     nq = min(a.nq, 10000)   # a bounded sample of the step (c5's step is 1M queries)
@@ -260,6 +298,8 @@ def run_reference(a, rank, world):
     ti, td = po.bruteforce(X, Q[:nt], a.k, a.metric)
     # origin ids == row numbers of X; internal ids are NOT (a racy parallel insert numbers points in arrival order)
     rid, rball = recall_stats(res[0][:nt], res[1][:nt], res[4][:nt], ti, td)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, res[0], res[1], res[4])
     line = {
         "impl": "reference", "metric": "queries/sec @ recall@10", "value": qps, "unit": "queries/s", "n_gpus": a.gpus,
         "steps": a.steps, "warmup": a.warmup, "ms_per_step": dt / a.steps * 1e3, "higher_is_better": True,
@@ -344,7 +384,8 @@ def run_ours(a, rank, world, local_rank):
     GSTEP, NGRP = 2, 3
     out_grp = [torch.empty((GSTEP, nq, a.k, 16), dtype=torch.uint8, device="cuda") for _ in range(NGRP)]   # Neighbour_api[nq][k] x GSTEP
     out_dev = [out_grp[0][0]]                       # kernel-only timings and the single-GPU path write here
-    cnt_dev = torch.empty((nq,), dtype=torch.int32, device="cuda")
+    cnt_grp = torch.empty((NGRP, GSTEP, nq), dtype=torch.int32, device="cuda")   # answer counts, one row per answer buffer
+    cnt_dev = cnt_grp[0][0]
     same_shards = (not a.strong) or a.nq % world == 0
     gather_grp = [torch.empty((world, GSTEP, nq, a.k, 16), dtype=torch.uint8, device="cuda") for _ in range(NGRP)] if multi and same_shards else None
     gather_dev = gather_grp
@@ -364,10 +405,11 @@ def run_ours(a, rank, world, local_rank):
         open_group[0] = None
 
     def step_device(i, sync=False):
-        g, j = (i // GSTEP) % NGRP, i % GSTEP
+        g, j = step_slot(i, GSTEP, NGRP)
         if gather_grp is not None and j == 0 and i >= GSTEP * NGRP:
             stream.wait_event(ev_gath[g])          # the all-gather that read this group NGRP groups ago has finished
-        ms = h.search_device(q_dev[i % NB].data_ptr(), nq, a.k, a.ef, out_grp[g][j].data_ptr(), cnt_dev.data_ptr(), sync=sync)
+        ms = h.search_device(q_dev[i % NB].data_ptr(), nq, a.k, a.ef, out_grp[g][j].data_ptr(), cnt_grp[g][j].data_ptr(),
+                             sync=sync)
         if gather_grp is not None:
             h.stream_wait_last(gstream.cuda_stream)   # the gather stream waits for every launch of the group
             open_group[0] = g
@@ -422,6 +464,11 @@ def run_ours(a, rank, world, local_rank):
     note('device-timed loop done')
     if h.check_status() != 0:
         raise RuntimeError("visited table overflow during the timed region")
+    last_step = None
+    if a.dump_outputs and rank == 0:
+        # rank 0's answers of the last timed step, before the launches below reuse out_grp[0][0] and cnt_dev
+        g, j = step_slot(a.steps - 1, GSTEP, NGRP)
+        last_step = (out_grp[g][j].cpu().numpy(), cnt_grp[g][j].cpu().numpy())
     clocks = clk.summary()
     # per-launch kernel duration (CUDA events inside the library, around the kernel alone)
     kms = [h.search_device(q_dev[i % NB].data_ptr(), nq, a.k, a.ef, out_dev[0].data_ptr(), cnt_dev.data_ptr(), sync=True)
@@ -551,6 +598,9 @@ def run_ours(a, rank, world, local_rank):
 
     if rank != 0:
         return
+    if last_step is not None:
+        rec, cnt = last_step
+        dump_outputs(a.dump_outputs, *decode_records(rec), cnt)
     peak, peak_src = measured_peak_gbs()
     step_ms = dev_ms / a.steps                      # average launch duration over the timed region (launches overlap pairwise)
     achieved = bytes_per_query * nq / (step_ms / 1e3) / 1e9
@@ -612,7 +662,6 @@ def cpu_baseline(a, h, Q):
     mode (Rust-std heaps, AVX2-shaped sums), one query per task over all host threads like rayon par_iter."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import pyoracle as po
-    po.build()
     logical = os.cpu_count() or 1
     lv, rk, og, entry = h.export_points()
     # the graph is imported by ONE thread: interleave its pages over the NUMA nodes, as the reference's own
@@ -662,6 +711,7 @@ _REAL_STDOUT = [1]
 
 
 def main():
+    sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
     a = parse()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
