@@ -494,6 +494,25 @@ int hnsw_b200_insert_flat(void* h, const void* vecs, uint64_t n, uint64_t dim, c
   return pass(ix, ix->insert_batch(vecs, n, dim, nullptr, ids, levels));
 }
 
+// one device's answers for queries [first, first + count) into the caller's arrays.  The kernel fills the slots beyond a
+// query's count with (~0, +inf, INVALID_ID): plain field copies
+static void unpack_answers(const Index* rx, const NeighbourOut* tmp, const int32_t* cnts, size_t first, size_t count,
+                           uint64_t knbn, uint64_t* out_ids, float* out_dist, uint32_t* out_internal, int32_t* out_pid,
+                           int32_t* out_counts) {
+  memcpy(out_counts + first, cnts, count * sizeof(int32_t));
+  const uint64_t tot = count * knbn, o0 = first * knbn;
+  for (uint64_t s = 0; s < tot; ++s) out_ids[o0 + s] = tmp[s].origin;
+  for (uint64_t s = 0; s < tot; ++s) out_dist[o0 + s] = tmp[s].dist;
+  if (out_internal)
+    for (uint64_t s = 0; s < tot; ++s) out_internal[o0 + s] = tmp[s].internal;
+  if (out_pid)  // PointId(level, rank), hnsw.rs:46
+    for (uint64_t s = 0; s < tot; ++s) {
+      const uint32_t it = tmp[s].internal;
+      out_pid[2 * (o0 + s)] = it != hb::INVALID_ID ? (int32_t)rx->h_level[it] : -1;
+      out_pid[2 * (o0 + s) + 1] = it != hb::INVALID_ID ? rx->h_rank[it] : -1;
+    }
+}
+
 int hnsw_b200_search_flat(const void* h, const void* queries, uint64_t nq, uint64_t dim, uint64_t knbn,
                           uint64_t ef_search, int filter_mode, const uint64_t* filter_ids, uint64_t nfilter,
                           hnsw_b200_filter_fn fn, void* ctx, uint64_t* out_ids, float* out_dist,
@@ -516,19 +535,44 @@ int hnsw_b200_search_flat(const void* h, const void* queries, uint64_t nq, uint6
     Index::CtxLease lease(rx);  // the answers stay in the context's pinned buffer until they are unpacked below
     int r = rx->search_host_staged(lease.c, (const char*)queries + first * qrow, nullptr, count, (int)dim, knbn, ef_search, fb, &tmp, &cnts);
     if (r) return r;
-    memcpy(out_counts + first, cnts, count * sizeof(int32_t));
-    // the kernel fills the slots beyond a query's count with (~0, +inf, INVALID_ID): plain field copies
-    const uint64_t tot = count * knbn, o0 = first * knbn;
-    for (uint64_t s = 0; s < tot; ++s) out_ids[o0 + s] = tmp[s].origin;
-    for (uint64_t s = 0; s < tot; ++s) out_dist[o0 + s] = tmp[s].dist;
-    if (out_internal)
-      for (uint64_t s = 0; s < tot; ++s) out_internal[o0 + s] = tmp[s].internal;
-    if (out_pid)  // PointId(level, rank), hnsw.rs:46
-      for (uint64_t s = 0; s < tot; ++s) {
-        const uint32_t it = tmp[s].internal;
-        out_pid[2 * (o0 + s)] = it != hb::INVALID_ID ? (int32_t)rx->h_level[it] : -1;
-        out_pid[2 * (o0 + s) + 1] = it != hb::INVALID_ID ? rx->h_rank[it] : -1;
-      }
+    unpack_answers(rx, tmp, cnts, first, count, knbn, out_ids, out_dist, out_internal, out_pid, out_counts);
+    return 0;
+  };
+  return pass(ix, use_shards(ix, nq) ? ix->for_each_shard(nq, run) : run(ix, 0, nq));
+}
+
+int hnsw_b200_search_flat_filters(const void* h, const void* queries, uint64_t nq, uint64_t dim, uint64_t knbn,
+                                  uint64_t ef_search, const uint64_t* filter_offsets, const uint64_t* filter_ids,
+                                  uint64_t* out_ids, float* out_dist, uint32_t* out_internal, int32_t* out_pid,
+                                  int32_t* out_counts) {
+  HB_HS(h);
+  if (nq == 0) return 0;
+  if (!queries || !out_ids || !out_dist || !out_counts || !filter_offsets) return set_err("search_flat_filters: NULL array");
+  if (knbn == 0) return set_err("search_flat_filters: knbn must be positive");
+  if (filter_offsets[0] != 0) return set_err("search_flat_filters: filter_offsets[0] must be 0");
+  for (uint64_t i = 0; i < nq; ++i)
+    if (filter_offsets[i + 1] < filter_offsets[i])
+      return set_err("search_flat_filters: filter_offsets decrease at query " + std::to_string(i));
+  if (filter_offsets[nq] != 0 && !filter_ids) return set_err("search_flat_filters: filter_ids is NULL");
+  for (uint64_t i = 0; i < nq; ++i)
+    for (uint64_t j = filter_offsets[i] + 1; j < filter_offsets[i + 1]; ++j)
+      if (filter_ids[j] < filter_ids[j - 1])
+        return set_err("search_flat_filters: the ids of query " + std::to_string(i) + " are not ascending");
+  // translated once, on this device; replicas hold the same internal ids and read their shard's descriptors
+  Index::QueryFilterSet qf;
+  int r = pass(ix, ix->make_query_filters(nq, filter_offsets, filter_ids, qf));
+  if (r) return r;
+  const size_t qrow = (size_t)dim * ix->es;
+  const hb::QueryFilter* desc = qf.desc.data();
+  const uint32_t* pay = qf.payload.data();
+  auto run = [=](Index* rx, size_t first, size_t count) -> int {
+    const NeighbourOut* tmp = nullptr;
+    const int32_t* cnts = nullptr;
+    Index::CtxLease lease(rx);
+    int rr = rx->search_host_staged(lease.c, (const char*)queries + first * qrow, nullptr, count, (int)dim, knbn, ef_search,
+                                    nullptr, &tmp, &cnts, desc + first, pay);
+    if (rr) return rr;
+    unpack_answers(rx, tmp, cnts, first, count, knbn, out_ids, out_dist, out_internal, out_pid, out_counts);
     return 0;
   };
   return pass(ix, use_shards(ix, nq) ? ix->for_each_shard(nq, run) : run(ix, 0, nq));

@@ -9,7 +9,11 @@
 //     and keeps expanding, until C is empty.
 // So here C is a real queue: an unsorted array of keys per warp in global memory, pop = warp-wide min scan
 // (consumed entries are overwritten with ~0).  W is the same sorted shared-memory array as elsewhere.
-// The FilterT predicate (filter.rs:7-24) is a device bitmap over internal ids, materialised by the host.
+// The FilterT predicate (filter.rs:7-24) is a policy (Pol below), tested at four sites: the retain pass over W, the
+// per-candidate pass mask, the W.n == 1 entry-point check and the post-filter after truncation.
+//   * BatchBits: one device bitmap over internal ids for the whole batch, materialised by the host;
+//   * PerQuery: query qi's own filter (QueryFilter, kernels.h), loaded when the warp picks the query up: a bitmap, or an
+//     ascending list of internal ids that each lane binary-searches for its own id.
 #include "kernels.h"
 #include "search_core.cuh"
 
@@ -19,9 +23,40 @@ __device__ __forceinline__ bool filter_pass(const uint32_t* bits, uint32_t id) {
   return (__ldg(bits + (id >> 5)) >> (id & 31)) & 1u;
 }
 
-template <class Op, int CH, int U>
+struct BatchBits {
+  const SearchParams& p;  // reads p.filter_bits where it is used, as the kernel did before it took a policy
+  __device__ __forceinline__ explicit BatchBits(const SearchParams& sp) : p(sp) {}
+  __device__ __forceinline__ void load(const SearchParams&, uint32_t) {}
+  __device__ __forceinline__ bool pass(uint32_t id) const { return filter_pass(p.filter_bits, id); }
+};
+
+struct PerQuery {
+  const uint32_t* data;  // this query's payload
+  uint32_t len;
+  bool bitmap;
+  __device__ __forceinline__ explicit PerQuery(const SearchParams&) : data(nullptr), len(0), bitmap(false) {}
+  // every lane loads the same descriptor (one 16-byte load)
+  __device__ __forceinline__ void load(const SearchParams& p, uint32_t qi) {
+    const uint4 d = __ldg(reinterpret_cast<const uint4*>(p.qfilters + qi));
+    data = p.qpayload + d.x;
+    len = d.y;
+    bitmap = d.z == QF_BITMAP;
+  }
+  __device__ __forceinline__ bool pass(uint32_t id) const {
+    if (bitmap) return filter_pass(data, id);
+    uint32_t lo = 0, hi = len;  // first position with data[pos] >= id
+    while (lo < hi) {
+      const uint32_t mid = (lo + hi) >> 1;
+      if (__ldg(data + mid) < id) lo = mid + 1;
+      else hi = mid;
+    }
+    return lo < len && __ldg(data + lo) == id;
+  }
+};
+
+template <class Op, int CH, int U, class Pol>
 __device__ __forceinline__ void search_layer_filtered(const GraphView& g, const WarpSmem& s, Visited& vis, SortedQueue& W,
-                                                      uint64_t* cbuf, uint32_t ccap, const uint32_t* fbits, uint32_t ep,
+                                                      uint64_t* cbuf, uint32_t ccap, const Pol& filt, uint32_t ep,
                                                       int ef, int layer, Stats& st, bool& overflow) {
   const int lane = lane_id();
   const uint4* vec4 = reinterpret_cast<const uint4*>(g.vec);
@@ -82,7 +117,7 @@ __device__ __forceinline__ void search_layer_filtered(const GraphView& g, const 
         bool keep = false;
         if (i < W.n) {
           v = W.w[i];
-          keep = filter_pass(fbits, key_id(v));
+          keep = filt.pass(key_id(v));
         }
         const unsigned m = __ballot_sync(FULL, keep);
         __syncwarp();
@@ -113,7 +148,7 @@ __device__ __forceinline__ void search_layer_filtered(const GraphView& g, const 
         st.evals += cnt;
         const uint32_t my_id = lane < cnt ? s.cand_id[lane] : 0u;
         const uint64_t key = lane < cnt ? make_key(Op::post(s.cand_d[lane]), my_id) : ~0ull;
-        const bool my_pass = lane < cnt && filter_pass(fbits, my_id);
+        const bool my_pass = lane < cnt && filt.pass(my_id);
         const unsigned passmask = __ballot_sync(FULL, my_pass);
         for (int j = 0; j < cnt; ++j) {  // strictly in list order: the accept rule sees the W of that moment
           if (W.n == 0) {                // 1019-1024
@@ -130,7 +165,7 @@ __device__ __forceinline__ void search_layer_filtered(const GraphView& g, const 
             if (lane == 0) __stcg(cbuf + cn, kj);  // 1035-1036: every accepted candidate goes to C
             cn += 1;
             if ((passmask >> j) & 1u) {  // 1040-1049
-              if (W.n == 1 && !filter_pass(fbits, key_id(W.w[0]))) W.n = 0;
+              if (W.n == 1 && !filt.pass(key_id(W.w[0]))) W.n = 0;
               __syncwarp();
               W.insert(kj);  // push, and pop the farthest when over ef (1051-1053)
             }
@@ -148,7 +183,7 @@ __device__ __forceinline__ void search_layer_filtered(const GraphView& g, const 
   }
 }
 
-template <class Op, int CH, int U>
+template <class Op, int CH, int U, class Pol>
 __global__ void __launch_bounds__(SEARCH_THREADS) search_filter_kernel(SearchParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -167,12 +202,14 @@ __global__ void __launch_bounds__(SEARCH_THREADS) search_filter_kernel(SearchPar
   SortedQueue W;
   Stats st{0, 0, 0};
   const uint4* vec4 = reinterpret_cast<const uint4*>(g.vec);
+  Pol filt(p);
 
   for (;;) {
     uint32_t qi = 0;
     if (lane == 0) qi = atomicAdd(p.work_counter, 1u);
     qi = __shfl_sync(FULL, qi, 0);
     if (qi >= p.nq) break;
+    filt.load(p, qi);
     stage_row_bytes(s.q4, reinterpret_cast<const char*>(p.queries) + (size_t)qi * p.q_stride_bytes, p.q_bytes, g.d4 * 16);
     int count = 0;
     bool overflow = false;
@@ -218,7 +255,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS) search_filter_kernel(SearchPar
         }
         pivot = new_pivot;
       }
-      search_layer_filtered<Op, CH, U>(g, s, vis, W, cbuf, p.ccap, p.filter_bits, pivot, p.ef, p.layer0, st, overflow);
+      search_layer_filtered<Op, CH, U, Pol>(g, s, vis, W, cbuf, p.ccap, filt, pivot, p.ef, p.layer0, st, overflow);
       count = min(p.k, min(p.ef, W.n));  // hnsw.rs:1547
     }
     if (overflow) {
@@ -234,7 +271,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS) search_filter_kernel(SearchPar
       bool keep = false;
       if (j < count) {
         key = W.w[j];
-        keep = filter_pass(p.filter_bits, key_id(key));
+        keep = filt.pass(key_id(key));
       }
       const unsigned m = __ballot_sync(FULL, keep);
       if (keep) {
@@ -255,13 +292,13 @@ __global__ void __launch_bounds__(SEARCH_THREADS) search_filter_kernel(SearchPar
   }
 }
 
-template <class Op>
+template <class Op, class Pol>
 static cudaError_t launch_filter_for_op(const SearchParams& p, int grid, size_t smem, cudaStream_t st, bool query_only,
                                         int* blocks_per_sm) {
   const int ch = p.g.d4 / 8;
 #define HB_LAUNCH(CHV, UV)                                                                              \
   do {                                                                                                  \
-    auto kern = search_filter_kernel<Op, CHV, UV>;                                                      \
+    auto kern = search_filter_kernel<Op, CHV, UV, Pol>;                                                 \
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
     if (e != cudaSuccess) return e;                                                                     \
     if (blocks_per_sm) {                                                                                \
@@ -282,7 +319,8 @@ cudaError_t launch_search_filtered(const SearchParams& p, int metric, int dtype,
                                    bool query_only, int* blocks_per_sm) {
   return dispatch_op(metric, dtype, [&](auto tag) -> cudaError_t {
     using Op = typename decltype(tag)::type;
-    return launch_filter_for_op<Op>(p, grid, smem, st, query_only, blocks_per_sm);
+    if (p.qfilters) return launch_filter_for_op<Op, PerQuery>(p, grid, smem, st, query_only, blocks_per_sm);
+    return launch_filter_for_op<Op, BatchBits>(p, grid, smem, st, query_only, blocks_per_sm);
   });
 }
 

@@ -107,6 +107,7 @@ Index::~Index() {
     if (c.stream) cudaStreamSynchronize(c.stream);
     cudaFree(c.vis.tab); cudaFree(c.vis.epoch); cudaFree(c.fvis.tab); cudaFree(c.fvis.epoch); cudaFree(c.d_counter); cudaFree(c.d_status);
     cudaFree(c.d_q); cudaFree(c.d_out); cudaFree(c.d_cnt); cudaFree(c.d_fbits); cudaFree(c.d_cbuf);
+    cudaFree(c.d_qf);
     if (c.h_pin) cudaFreeHost(c.h_pin);
     if (c.h_res) cudaFreeHost(c.h_res);
     if (c.fork) cudaEventDestroy(c.fork);
@@ -288,6 +289,7 @@ int Index::check_insert_fit() {
 
 // forget the points [keep, n): they were stored but never linked (a failed insert call)
 void Index::rollback_points(size_t keep) {
+  invalidate_origin_table();
   n = keep;
   h_level.resize(keep);
   h_plevel.resize(keep);
@@ -373,6 +375,7 @@ int Index::insert_batch(const void* vecs, size_t n_new, size_t stride, const voi
   if ((r = ensure_points(n + n_new))) return r;
   if ((r = ensure_upper(n_ul + need_ul + 2 * MAX_LAYERS))) return r;
   const size_t first = n;
+  invalidate_origin_table();
   h_level.resize(first + n_new);
   h_plevel.resize(first + n_new);
   h_rank.resize(first + n_new);
@@ -519,6 +522,7 @@ int Index::import_graph(const void* vecs, size_t n_new, int d, const uint64_t* o
   h_level.assign(levels, levels + n_new);
   h_plevel = pl;
   h_rank.resize(n_new);
+  invalidate_origin_table();  // also the path of a dump load (load_dump)
   h_origin.assign(origin, origin + n_new);
   h_upoff.resize(n_new);
   for (int l = 0; l < MAX_LAYERS; ++l) layer_count[l] = 0;
@@ -641,7 +645,8 @@ int Index::stream_wait_last(cudaStream_t s) {
 }
 
 int Index::search_on_ctx(SearchCtx& c, const void* d_queries, size_t nq, size_t k, size_t ef_arg, const uint32_t* d_filter_bits,
-                         NeighbourOut* d_out, int32_t* d_counts, bool sync, float* kernel_ms) {
+                         NeighbourOut* d_out, int32_t* d_counts, bool sync, float* kernel_ms, const QueryFilter* d_qf,
+                         const uint32_t* d_qpay) {
   if (k == 0) return fail("knbn must be positive");
   if (poisoned_) return fail(poison_msg_);
   cudaStream_t st = c.stream;
@@ -666,9 +671,11 @@ int Index::search_on_ctx(SearchCtx& c, const void* d_queries, size_t nq, size_t 
   p.out_nb = d_out;
   p.out_count = d_counts;
   p.filter_bits = d_filter_bits;
+  p.qfilters = d_qf;
+  p.qpayload = d_qpay;
   p.stats = stats_on_ ? d_stats_ : nullptr;
   p.status = c.d_status;
-  const bool filtered = d_filter_bits != nullptr;
+  const bool filtered = d_filter_bits != nullptr || d_qf != nullptr;
   // kernel choice: lean (search_lean.cuh) whenever it applies, else the generic warp kernel (search.cu / filter.cu)
   // tie mode "std" (search_std.cu): the reference's heaps replayed literally, unfiltered searches only
   const bool stdtie = tie_std_ && !filtered;
@@ -691,7 +698,7 @@ int Index::search_on_ctx(SearchCtx& c, const void* d_queries, size_t nq, size_t 
   int bps = 0;
   {
     std::lock_guard<std::mutex> lk(occ_mu_);
-    const auto key = std::make_tuple(stdtie ? 4 : (lean ? 3 : (int)filtered), (lean ? p.q_smem : p.q_kind) * 64 + wpb, p.g.d4, smem);
+    const auto key = std::make_tuple(stdtie ? 4 : (lean ? 3 : (d_qf ? 5 : (int)filtered)), (lean ? p.q_smem : p.q_kind) * 64 + wpb, p.g.d4, smem);
     auto it = occ_cache_.find(key);
     if (it != occ_cache_.end()) {
       bps = it->second;
@@ -770,7 +777,7 @@ static const void* device_view_of_host(const void* p) {
 // gathered into the index's own pinned staging buffer first (the only host-side copy), which the kernel then reads
 // the same way.  zero_copy_ = false (env HNSW_B200_ZERO_COPY=0) restores explicit H2D / D2H copies.
 int Index::search_host_begin(int ci, const void* queries, const void* const* rows, size_t nq, int d, size_t k, size_t ef,
-                             const uint32_t* filter_bits_host) {
+                             const uint32_t* filter_bits_host, const QueryFilter* qdesc, const uint32_t* qpay) {
   SearchCtx& c = ctx_[ci];
   cudaStream_t st = c.stream;
   c.pend = SearchCtx::Pending();
@@ -848,15 +855,36 @@ int Index::search_host_begin(int ci, const void* queries, const void* const* row
     HB_CUDA(cudaMemcpyAsync(c.d_fbits, filter_bits_host, fb, cudaMemcpyHostToDevice, st));
     dfb = (const uint32_t*)c.d_fbits;
   }
+  const QueryFilter* dqf = nullptr;
+  const uint32_t* dqpay = nullptr;
+  if (qdesc) {  // per-query filters: this batch's descriptors, re-based, then the payload range they name
+    const size_t words = (n + 31) / 32;
+    size_t lo = SIZE_MAX, hi = 0;
+    for (size_t i = 0; i < nq; ++i) {
+      lo = std::min<size_t>(lo, qdesc[i].off);
+      hi = std::max<size_t>(hi, (size_t)qdesc[i].off + (qdesc[i].form == QF_BITMAP ? words : qdesc[i].len));
+    }
+    std::vector<QueryFilter> rb(qdesc, qdesc + nq);
+    for (QueryFilter& q : rb) q.off -= (uint32_t)lo;
+    const size_t db = nq * sizeof(QueryFilter), pb = (hi - lo) * 4;
+    if ((r = ensure_scratch(&c.d_qf, &c.d_qf_bytes, db + pb, st))) return r;
+    // pageable sources: the calls return once the bytes are staged, so rb may go out of scope
+    HB_CUDA(cudaMemcpyAsync(c.d_qf, rb.data(), db, cudaMemcpyHostToDevice, st));
+    if (pb) HB_CUDA(cudaMemcpyAsync((char*)c.d_qf + db, qpay + lo, pb, cudaMemcpyHostToDevice, st));
+    dqf = (const QueryFilter*)c.d_qf;
+    dqpay = (const uint32_t*)((char*)c.d_qf + db);
+  }
   // one enqueue (copies if any, kernel, status); search_host_finish synchronises once and takes the slow path (a visited
   // table overflowed: grow and re-run) only when the status says so
   c.pend.d_queries = d_queries;
   c.pend.dfb = dfb;
+  c.pend.dqf = dqf;
+  c.pend.dqpay = dqpay;
   c.pend.k_out = k_out;
   c.pend.k_cnt = k_cnt;
   c.pend.direct = dv != nullptr;
   c.pend.enqueued = true;
-  if ((r = search_on_ctx(c, d_queries, nq, k, ef, dfb, k_out, k_cnt, false, nullptr))) return r;
+  if ((r = search_on_ctx(c, d_queries, nq, k, ef, dfb, k_out, k_cnt, false, nullptr, dqf, dqpay))) return r;
   if (!c.pend.direct) {
     HB_CUDA(cudaMemcpyAsync(hout, c.d_out, out_bytes, cudaMemcpyDeviceToHost, st));
     HB_CUDA(cudaMemcpyAsync(hcnt, c.d_cnt, cnt_bytes, cudaMemcpyDeviceToHost, st));
@@ -877,7 +905,8 @@ int Index::search_host_finish(int ci, const NeighbourOut** out, const int32_t** 
   if (*p.hstatus == 0) return 0;
   HB_CUDA(cudaMemsetAsync(c.d_status, 0, sizeof(int), st));
   int r;
-  if ((r = search_on_ctx(c, p.d_queries, p.nq, p.k, p.ef, p.dfb, p.k_out, p.k_cnt, true, nullptr))) return r;  // grows the tables
+  if ((r = search_on_ctx(c, p.d_queries, p.nq, p.k, p.ef, p.dfb, p.k_out, p.k_cnt, true, nullptr, p.dqf, p.dqpay)))
+    return r;  // grows the tables
   if (!p.direct) {
     HB_CUDA(cudaMemcpyAsync(p.hout, c.d_out, p.out_bytes, cudaMemcpyDeviceToHost, st));
     HB_CUDA(cudaMemcpyAsync(p.hcnt, c.d_cnt, p.cnt_bytes, cudaMemcpyDeviceToHost, st));
@@ -887,10 +916,11 @@ int Index::search_host_finish(int ci, const NeighbourOut** out, const int32_t** 
 }
 
 int Index::search_host_staged(int ci, const void* queries, const void* const* rows, size_t nq, int d, size_t k, size_t ef,
-                              const uint32_t* filter_bits_host, const NeighbourOut** out, const int32_t** counts) {
+                              const uint32_t* filter_bits_host, const NeighbourOut** out, const int32_t** counts,
+                              const QueryFilter* qdesc, const uint32_t* qpay) {
   *out = nullptr;
   *counts = nullptr;
-  int r = search_host_begin(ci, queries, rows, nq, d, k, ef, filter_bits_host);
+  int r = search_host_begin(ci, queries, rows, nq, d, k, ef, filter_bits_host, qdesc, qpay);
   if (r) return r;
   return search_host_finish(ci, out, counts);
 }
@@ -920,6 +950,91 @@ int Index::make_filter_bits(int mode, const uint64_t* sorted_ids, size_t nids, i
     }
     if (pass) bits[i >> 5] |= 1u << (i & 31);
   }
+  return 0;
+}
+
+// Per-query filters.  Origin ids are translated through origin_table_, (origin, internal) sorted once per change of
+// h_origin: a short list binary-searches it (resuming where the previous id was found), a long one walks it in step.
+// Two passes over contiguous chunks of queries on host threads: the first counts each query's internal ids, which fixes
+// its form and its place in the payload (so the size limit is checked exactly, before anything is allocated); the
+// second translates again and writes the query's list or bitmap in place.
+int Index::make_query_filters(size_t nq, const uint64_t* offsets, const uint64_t* ids, QueryFilterSet& out) const {
+  {
+    std::lock_guard<std::mutex> lk(origin_mu_);
+    if (!origin_table_ok_) {
+      origin_table_.resize(n);
+      for (size_t i = 0; i < n; ++i) origin_table_[i] = {h_origin[i], (uint32_t)i};
+      std::sort(origin_table_.begin(), origin_table_.end());
+      origin_table_ok_ = true;
+    }
+  }
+  // the table changes only under the index's exclusive lock, which no search holds: read it without origin_mu_
+  const std::pair<uint64_t, uint32_t>* T = origin_table_.data();
+  const size_t nt = origin_table_.size(), words = (n + 31) / 32;
+  unsigned lg = 1;
+  while (lg < 63 && ((size_t)1 << lg) < nt) ++lg;
+  // calls range(lo, hi) for every run T[lo .. hi) of points whose origin id is in query q's list
+  auto translate = [&](size_t q, auto&& range) {
+    const uint64_t* a = ids + offsets[q];
+    const size_t len = offsets[q + 1] - offsets[q];
+    const bool walk = len * lg >= nt;
+    size_t pos = 0;
+    for (size_t j = 0; j < len; ++j) {
+      if (j && a[j] == a[j - 1]) continue;
+      size_t end;
+      if (walk) {
+        while (pos < nt && T[pos].first < a[j]) ++pos;
+        for (end = pos; end < nt && T[end].first == a[j];) ++end;
+      } else {
+        pos = std::lower_bound(T + pos, T + nt, std::make_pair(a[j], (uint32_t)0)) - T;
+        end = std::upper_bound(T + pos, T + nt, std::make_pair(a[j], UINT32_MAX)) - T;
+      }
+      if (end > pos) range(pos, end);
+      pos = end;
+    }
+  };
+  const size_t hw = std::max(1u, std::thread::hardware_concurrency());
+  const size_t nth = std::max<size_t>(1, std::min<size_t>(std::min<size_t>(hw, 32), nq / 16));
+  auto parallel = [&](const std::function<void(size_t, size_t)>& fn) {  // fn(first query, end) per chunk
+    if (nth == 1) return fn(0, nq);
+    std::vector<std::thread> th;
+    for (size_t t = 0; t < nth; ++t) th.emplace_back(fn, nq * t / nth, nq * (t + 1) / nth);
+    for (auto& x : th) x.join();
+  };
+  out.desc.assign(nq, QueryFilter{0, 0, QF_LIST, 0});
+  parallel([&](size_t q0, size_t q1) {
+    for (size_t q = q0; q < q1; ++q) {
+      size_t c = 0;
+      translate(q, [&](size_t lo, size_t hi) { c += hi - lo; });
+      out.desc[q].len = (uint32_t)c;  // c <= n < 2^32
+      out.desc[q].form = qf_use_bitmap(c, n) ? QF_BITMAP : QF_LIST;
+    }
+  });
+  size_t total = 0;
+  for (QueryFilter& d : out.desc) {
+    if (total > UINT32_MAX) break;
+    d.off = (uint32_t)total;
+    total += d.form == QF_BITMAP ? words : d.len;
+  }
+  if (total > UINT32_MAX)
+    return fail("per-query filters: the packed filters need more than 2^32 - 1 32-bit words");
+  out.payload.assign(total, 0u);
+  parallel([&](size_t q0, size_t q1) {
+    for (size_t q = q0; q < q1; ++q) {
+      uint32_t* dst = out.payload.data() + out.desc[q].off;
+      if (out.desc[q].form == QF_BITMAP) {
+        translate(q, [&](size_t lo, size_t hi) {
+          for (size_t i = lo; i < hi; ++i) dst[T[i].second >> 5] |= 1u << (T[i].second & 31);
+        });
+      } else {
+        size_t c = 0;
+        translate(q, [&](size_t lo, size_t hi) {
+          for (size_t i = lo; i < hi; ++i) dst[c++] = T[i].second;
+        });
+        std::sort(dst, dst + c);
+      }
+    }
+  });
   return 0;
 }
 
@@ -1111,6 +1226,7 @@ int Index::blob_info(int i, void** p, uint64_t* bytes) const {
 
 int Index::blob_commit() {
   cudaSetDevice(device);
+  invalidate_origin_table();
   h_level.resize(n);
   h_plevel.resize(n);
   h_origin.resize(n);

@@ -101,8 +101,10 @@ class Index {
   int search_host(const void* queries, const void* const* rows, size_t nq, int d, size_t k, size_t ef,
                   const uint32_t* filter_bits_host, NeighbourOut* out, int32_t* counts);
   // same on context c (a CtxLease), answers left in the context's pinned buffer (valid until the lease ends)
+  // qdesc / qpay: per-query filters instead of filter_bits_host (QueryFilterSet below; qdesc[i] is query i's, its offset
+  // counts from qpay, which only the range those nq descriptors name is read of)
   int search_host_begin(int c, const void* queries, const void* const* rows, size_t nq, int d, size_t k, size_t ef,
-                        const uint32_t* filter_bits_host);
+                        const uint32_t* filter_bits_host, const QueryFilter* qdesc = nullptr, const uint32_t* qpay = nullptr);
   int search_host_finish(int c, const NeighbourOut** out, const int32_t** counts);
   // submitted-but-not-waited host searches: anything that changes the graph waits for them (drain_pending)
   std::atomic<int> pending_{0};
@@ -110,12 +112,23 @@ class Index {
     while (pending_.load() != 0) std::this_thread::yield();
   }
   int search_host_staged(int c, const void* queries, const void* const* rows, size_t nq, int d, size_t k, size_t ef,
-                         const uint32_t* filter_bits_host, const NeighbourOut** out, const int32_t** counts);
+                         const uint32_t* filter_bits_host, const NeighbourOut** out, const int32_t** counts,
+                         const QueryFilter* qdesc = nullptr, const uint32_t* qpay = nullptr);
   int search_device(const void* d_queries, size_t nq, size_t k, size_t ef, const uint32_t* d_filter_bits,
                     NeighbourOut* d_out, int32_t* d_counts, bool sync, float* kernel_ms);
   // filter materialisation: bit per internal id from a sorted origin-id list or a callback
   int make_filter_bits(int mode, const uint64_t* sorted_ids, size_t nids, int (*fn)(uint64_t, void*), void* ctx,
                        std::vector<uint32_t>& bits) const;
+  // One FilterT per query: query i admits the points whose origin id is in ids[offsets[i] .. offsets[i+1]) (ascending,
+  // repeats allowed; every point sharing an admitted origin id is admitted, ids not in the index are ignored).  Translated
+  // to internal ids and packed per query as a list or a bitmap (QueryFilter, kernels.h).  The caller validates the input.
+  // Searches with per-query filters always run the filtered kernel; tie mode "std" does not apply to them, as to batch
+  // filters.
+  struct QueryFilterSet {
+    std::vector<QueryFilter> desc;  // [nq], offsets into payload
+    std::vector<uint32_t> payload;
+  };
+  int make_query_filters(size_t nq, const uint64_t* offsets, const uint64_t* ids, QueryFilterSet& out) const;
 
   int export_layer(int layer, uint64_t* offsets, uint32_t* ids, float* dists, int64_t* total) const;
   int export_vectors(void* out) const;
@@ -174,14 +187,16 @@ class Index {
     unsigned int* d_counter = nullptr;
     int* d_status = nullptr;
     VisitedPool vis, fvis;  // unfiltered / filtered searches
-    void *d_q = nullptr, *d_out = nullptr, *d_cnt = nullptr, *d_fbits = nullptr, *d_cbuf = nullptr;
-    size_t d_q_bytes = 0, d_out_bytes = 0, d_cnt_bytes = 0, d_fbits_bytes = 0, d_cbuf_bytes = 0;
+    void *d_q = nullptr, *d_out = nullptr, *d_cnt = nullptr, *d_fbits = nullptr, *d_cbuf = nullptr, *d_qf = nullptr;
+    size_t d_q_bytes = 0, d_out_bytes = 0, d_cnt_bytes = 0, d_fbits_bytes = 0, d_cbuf_bytes = 0, d_qf_bytes = 0;
     void *h_pin = nullptr, *h_res = nullptr;  // pinned, mapped: query staging / answers
     size_t h_pin_bytes = 0, h_res_bytes = 0;
     bool busy = false;
     struct Pending {  // a host search enqueued by search_host_begin, completed by search_host_finish
       const void* d_queries = nullptr;
       const uint32_t* dfb = nullptr;
+      const QueryFilter* dqf = nullptr;  // per-query filters: descriptors and payload in d_qf
+      const uint32_t* dqpay = nullptr;
       NeighbourOut *k_out = nullptr, *hout = nullptr;
       int32_t *k_cnt = nullptr, *hcnt = nullptr, *hstatus = nullptr;
       size_t nq = 0, k = 0, ef = 0, out_bytes = 0, cnt_bytes = 0;
@@ -268,7 +283,8 @@ class Index {
   VisitedPool vis_;  // visited tables of the insert kernel (searches: SearchCtx)
   SearchCtx ctx_[NCTX + NASYNC];
   int search_on_ctx(SearchCtx& c, const void* d_queries, size_t nq, size_t k, size_t ef_arg, const uint32_t* d_filter_bits,
-                    NeighbourOut* d_out, int32_t* d_counts, bool sync, float* kernel_ms);
+                    NeighbourOut* d_out, int32_t* d_counts, bool sync, float* kernel_ms, const QueryFilter* d_qf = nullptr,
+                    const uint32_t* d_qpay = nullptr);
   std::mutex ctx_mu_;
   std::condition_variable ctx_cv_;
   std::mutex ticket_mu_, shard_mu_;
@@ -293,6 +309,17 @@ class Index {
   std::map<std::tuple<int, int, int, size_t>, int> occ_cache_;  // (filtered, queue kind, d4, smem) -> CTAs/SM
   void* d_mask_ = nullptr;
   size_t d_mask_bytes_ = 0;
+
+  // (origin id, internal id) sorted, for make_query_filters: built on first use, dropped wherever h_origin changes
+  mutable std::mutex origin_mu_;
+  mutable std::vector<std::pair<uint64_t, uint32_t>> origin_table_;
+  mutable bool origin_table_ok_ = false;
+  void invalidate_origin_table() {
+    std::lock_guard<std::mutex> lk(origin_mu_);
+    origin_table_ok_ = false;
+    origin_table_.clear();
+    origin_table_.shrink_to_fit();
+  }
 };
 
 }  // namespace hb

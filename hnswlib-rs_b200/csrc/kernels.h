@@ -27,6 +27,18 @@ struct NeighbourOut {
   uint32_t internal;
 };
 
+// One query's FilterT on the device.  form QF_LIST: payload[off .. off+len) are ascending internal ids; form QF_BITMAP:
+// payload[off .. off+ceil(n/32)) is a bit per internal id (len = ids admitted).  The host picks the bitmap when the list
+// would be at least as large (32 * len >= n), so a query never costs more than 4 bytes per admitted id.
+enum : uint32_t { QF_LIST = 0, QF_BITMAP = 1 };
+struct __align__(16) QueryFilter {
+  uint32_t off;  // in 32-bit words
+  uint32_t len;
+  uint32_t form;
+  uint32_t pad;
+};
+inline bool qf_use_bitmap(uint64_t len, uint64_t n) { return 32 * len >= n; }
+
 struct SearchParams {
   GraphView g;
   const void* queries;  // device, raw element bytes, row i at i * q_stride_bytes
@@ -40,7 +52,7 @@ struct SearchParams {
   unsigned int* work_counter;
   NeighbourOut* out_nb;  // [nq][k]
   int32_t* out_count;    // [nq]
-  const uint32_t* filter_bits;  // nullptr = no filter; bit per internal id
+  const uint32_t* filter_bits;  // nullptr = no batch filter; bit per internal id, one filter for every query
   unsigned long long* stats;    // nullptr or [3]: evals, expansions, adjacency ids read
   int* status;                  // set to 1 on visited-table overflow
   int smem_per_warp;
@@ -49,6 +61,9 @@ struct SearchParams {
   int q_kind;  // QueueSel kind
   uint64_t* cbuf;  // filtered search only: candidate queue C, [slots][ccap] keys
   uint32_t ccap;
+  // per-query filters (filter_bits == nullptr): query qi admits what qfilters[qi] describes in qpayload
+  const QueryFilter* qfilters;  // nullptr = none; [nq]
+  const uint32_t* qpayload;
 };
 
 // rows of up to 512 bytes are (partly) staged by TMA: STAGE_ROWS rows + an mbarrier per warp

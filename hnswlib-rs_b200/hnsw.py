@@ -85,6 +85,7 @@ def load_library():
     L.hnsw_b200_set_insert_batching.argtypes = [vp, C.c_uint32, C.c_uint32]
     L.hnsw_b200_insert_flat.argtypes = [vp, vp, u64, u64, vp, vp]
     L.hnsw_b200_search_flat.argtypes = [vp, vp, u64, u64, u64, u64, i32, vp, u64, FILTER_FN, vp, vp, vp, vp, vp, vp]
+    L.hnsw_b200_search_flat_filters.argtypes = [vp, vp, u64, u64, u64, u64, vp, vp, vp, vp, vp, vp, vp]
     L.hnsw_b200_search_device.argtypes = [vp, vp, u64, u64, u64, vp, vp, i32, vp]
     L.hnsw_b200_search_flat_submit.restype = i64
     L.hnsw_b200_search_flat_submit.argtypes = [vp, vp, u64, u64, u64, u64, vp, vp, vp, vp, vp]
@@ -131,6 +132,32 @@ def _p(a):
 
 class HnswError(RuntimeError):
     pass
+
+
+def pack_filters(filters, nq):
+    """One FilterT (id list) per query, packed for hnsw_b200_search_flat_filters: returns (offsets u64[nq + 1], ids u64),
+    query i admitting ids[offsets[i]:offsets[i + 1]].
+
+    filters is either a sequence of nq id sequences, each sorted here (as search_flat sorts its filter), or an
+    (offsets, ids) pair: a tuple of two numpy arrays whose first has nq + 1 entries.  The pair is checked to describe
+    ids exactly (offsets[0] == 0, offsets never decreasing, offsets[-1] == len(ids); ValueError otherwise: the library
+    cannot see the length of ids) and passed on unsorted (the library refuses a list that is not ascending).  A list is
+    never taken for a pair: pass per-query filters as a list to keep two numpy filters from reading as one pair."""
+    if (isinstance(filters, tuple) and len(filters) == 2 and all(isinstance(x, np.ndarray) for x in filters)
+            and len(filters[0]) == nq + 1):
+        offsets = np.ascontiguousarray(filters[0].reshape(-1), np.uint64)
+        ids = np.ascontiguousarray(filters[1].reshape(-1), np.uint64)
+        if offsets[0] != 0 or np.any(offsets[1:] < offsets[:-1]) or int(offsets[-1]) != len(ids):
+            raise ValueError(f"(offsets, ids) pair: offsets must start at 0, never decrease and end at len(ids) = {len(ids)}"
+                             " (to give per-query filters, pass them as a list)")
+        return offsets, ids
+    if len(filters) != nq:
+        raise ValueError(f"{len(filters)} filters for {nq} queries")
+    lists = [np.sort(np.asarray(f, np.uint64).reshape(-1)) for f in filters]
+    offsets = np.zeros(nq + 1, np.uint64)
+    offsets[1:] = np.cumsum([len(x) for x in lists], dtype=np.uint64)
+    ids = np.concatenate(lists) if lists else np.zeros(0, np.uint64)
+    return offsets, np.ascontiguousarray(ids, np.uint64)
 
 
 class Neighbour:
@@ -330,6 +357,31 @@ class Hnsw:
         self._chk(self._L.hnsw_b200_search_flat(self._h, _p(q), nq, d, int(knbn), int(ef), mode, _p(fids), nf, cb, None,
                                                 _p(o), _p(ds), _p(it), _p(pid), _p(cnt)))
         return o, ds, it, pid, cnt
+
+    def search_flat_filters(self, queries, knbn, ef, filters, with_internal=True, with_pid=True):
+        """hnsw_b200_search_flat_filters: search_flat with one id-list filter per query (pack_filters says what `filters`
+        may be).  Same outputs as search_flat."""
+        q = np.ascontiguousarray(queries, self.dtype)
+        nq, d = q.shape
+        offsets, ids = pack_filters(filters, nq)
+        o = np.empty((nq, knbn), np.uint64)
+        ds = np.empty((nq, knbn), np.float32)
+        it = np.empty((nq, knbn), np.uint32) if with_internal else None
+        pid = np.empty((nq, knbn, 2), np.int32) if with_pid else None
+        cnt = np.empty(nq, np.int32)
+        self._chk(self._L.hnsw_b200_search_flat_filters(self._h, _p(q), nq, d, int(knbn), int(ef), _p(offsets), _p(ids),
+                                                        _p(o), _p(ds), _p(it), _p(pid), _p(cnt)))
+        return o, ds, it, pid, cnt
+
+    def parallel_search_filter(self, datas, knbn, ef, filters):
+        """Batched counterpart of [search_filter(datas[i], knbn, ef, filters[i]) for i ...]: lists of Neighbour in input
+        order, one id-list filter per query."""
+        q = np.asarray([np.asarray(v, self.dtype) for v in datas], self.dtype)
+        if len(q) == 0:
+            return []
+        o, d, _, pid, cnt = self.search_flat_filters(q, knbn, ef, filters, with_internal=False)
+        return [[Neighbour(int(o[i, j]), float(d[i, j]), (int(pid[i, j, 0]), int(pid[i, j, 1]))) for j in range(cnt[i])]
+                for i in range(len(q))]
 
     def submit_flat(self, queries, knbn, ef, with_internal=True, with_pid=True):
         """hnsw_b200_search_flat_submit: enqueue a batch, return a ticket for wait_flat (up to 4 outstanding)"""

@@ -247,6 +247,20 @@ int hnsw_b200_search_flat(const void* h, const void* queries, uint64_t nq, uint6
                           hnsw_b200_filter_fn fn, void* ctx, uint64_t* out_ids, float* out_dist,
                           uint32_t* out_internal, int32_t* out_pid, int32_t* out_counts);
 
+/* One FilterT (sorted Vec<usize> of origin ids, filter.rs:11-15) per query: query i admits
+ * filter_ids[filter_offsets[i] .. filter_offsets[i+1]), ascending (repeats allowed).
+ * An empty range admits nothing.  Outputs as hnsw_b200_search_flat.  Sharded over replicas like it.
+ * filter_offsets has nq + 1 entries.  Every point whose origin id is listed is admitted (several points may share one);
+ * ids absent from the index are ignored.  Each query's list is packed for the device as ascending internal ids, or as
+ * a bitmap over the points when that is no larger (32 * ids >= points).  Tie mode "std" (hnsw_b200_set_tie_mode) does
+ * not apply, as with filter_mode != 0.  Refused (< 0, nothing launched, the handle stays usable): NULL arrays when
+ * nq > 0, filter_offsets[0] != 0, decreasing offsets, a list that is not ascending, packed filters of 2^32 words or
+ * more. */
+int hnsw_b200_search_flat_filters(const void* h, const void* queries, uint64_t nq, uint64_t dim, uint64_t knbn,
+                                  uint64_t ef_search, const uint64_t* filter_offsets, const uint64_t* filter_ids,
+                                  uint64_t* out_ids, float* out_dist, uint32_t* out_internal, int32_t* out_pid,
+                                  int32_t* out_counts);
+
 /* The same search (unfiltered; sharded over the replicas when hnsw_b200_replicate was called) split in two calls, so that ONE host thread keeps several batches in
  * flight: submit enqueues the batch and returns a ticket (>= 0; < 0 on error) at once, wait blocks until its answers
  * are in the arrays given to submit.  Up to 4 batches may be in flight per handle (a fifth submit blocks); the query and
